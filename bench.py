@@ -16,6 +16,7 @@ big20, big22, synthetic.
 
   python bench.py --gpus N --steps K --warmup W [--config C]      (torchrun launches N > 1)
   python bench.py --impl reference ...     the path's CPU port (oracle/) on the same config, all host threads, rank 0 only
+  python bench.py ... --dump-outputs DIR   also write what the last step of the first timed pass returned (step_outputs)
 """
 import argparse
 import json
@@ -250,6 +251,42 @@ def unit_count(name, ints):
     return None
 
 
+DUMP_CAP = 1 << 21        # elements kept of one dumped array (a dump of any config stays far below 64 MB)
+
+
+def step_outputs(prob, loss, res):
+    """What a caller of the timed path receives from one step, as host arrays (float32; integer outputs as float64): the loss,
+    the RenderResult fields and the parameter gradients.  An array of more than DUMP_CAP elements is flattened and replaced by a
+    fixed sample of DUMP_CAP of them (sorted indices from seed 0, a function of its size only), e.g. the 64 MB table gradient."""
+    import torch
+    field, shader, r = prob["field"], prob["shader"], prob["renderer"]
+    arrays = {"loss": loss.reshape(1), "colors": res.colors, "disparity": res.disparity, "depth": res.depth,
+              "first_oct_dis": res.first_oct_dis, "weights": res.weights, "idx_start_end": res.idx_start_end,
+              "edge_feats": res.edge_feats, "grad_feat_pool": field.feat_pool_.grad, "grad_field_mlp": field.mlp_.params_.grad,
+              "grad_shader_mlp": shader.mlp_.params_.grad, "grad_app_emb": r.app_emb_.grad}
+    out = {}
+    for name, t in arrays.items():
+        if t is None:
+            continue
+        t = t.detach()
+        if t.numel() > DUMP_CAP:
+            idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), DUMP_CAP))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        out[name] = a.astype(np.float64 if a.dtype.kind in "iu" else np.float32)
+    return out
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise RuntimeError(f"--dump-outputs: {total} bytes, over the 64 MB a dump may take")
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    print(f"bench.py: wrote {len(arrays)} arrays ({total / 1e6:.1f} MB) to {path}", file=sys.stderr)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -296,16 +333,16 @@ def run_ours(args):
         loss, res = train_step(prob, d_o, d_d, d_cam, d_gt, dist_sync, nxt)   # seen the steady-state peak before timing starts)
     barrier()
     clocks.rows.clear()                          # keep only samples taken under the timed regions
-    def timed_loop():
+    def timed_loop(capture):
         import gc
         gc.collect()
         gc.disable()                              # like timeit: no cyclic-GC pause inside the timed region
         try:
-            return _timed_loop()
+            return _timed_loop(capture)
         finally:
             gc.enable()
 
-    def _timed_loop():
+    def _timed_loop(capture):
         barrier()
         l0 = _lib.LAUNCHES
         ea, eb = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -320,7 +357,8 @@ def run_ours(args):
             w.append(round((time.perf_counter() - w0) * 1e3, 2))
         eb.record()
         barrier()
-        return ea.elapsed_time(eb), w, ns, nk, _lib.LAUNCHES - l0
+        out = step_outputs(prob, loss, res) if capture else None      # outside the timed window, before another step runs
+        return ea.elapsed_time(eb), w, ns, nk, _lib.LAUNCHES - l0, out
 
     # A step whose host wall time is far off the median (seen on fresh boxes: one NVML poll of the clock sampler
     # holding the driver lock for ~40 ms while the main thread launches) makes the whole K-step number a
@@ -336,8 +374,11 @@ def run_ours(args):
         return bool(bad)
 
     attempts, best = [], None
-    for _ in range(4):                            # at most three re-measurements, every attempt disclosed in `timing_attempts`
-        res = timed_loop()
+    for i in range(4):                            # at most three re-measurements, every attempt disclosed in `timing_attempts`
+        # the dump is the first pass's last step: its inputs (RNG position, octree votes so far) depend on the arguments only
+        res = timed_loop(capture=bool(args.dump_outputs) and rank == 0 and i == 0)
+        if i == 0:
+            dumped = res[5]
         outlier = stalled(res[1])
         attempts.append({"ms_per_step": res[0] / args.steps, "host_wall_ms_per_step": res[1], "rejected": bool(outlier)})
         if not outlier:
@@ -345,7 +386,7 @@ def run_ours(args):
             break
         if best is None or res[0] < best[0]:
             best = res                            # every attempt stalled: the least disturbed one stands, flagged as rejected
-    ms, walls, n_samples, n_kept, launches = best
+    ms, walls, n_samples, n_kept, launches, _ = best
     # ---- per-kernel CUDA-event trace over the same steps (separate loop: event pairs around every C-ABI call) --
     _lib.TRACE = []
     for _ in range(args.steps):
@@ -474,6 +515,8 @@ def run_ours(args):
         cpp = cpp_host_timing(args)
         if cpp is not None:
             line["cpp_host"] = cpp
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -749,7 +792,14 @@ def main():
                     help="march every batch at the start of its own Render (default: the next batch's march runs behind this step's backward)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last step of the first timed pass returned (loss, render outputs, parameter gradients) "
+                         "as DIR/<name>.npy; rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,5 +1,6 @@
 """Host-side logic of bench.py that must not break on the GPU box (no GPU needed): the `config` object both arms print, the governing
-rooflines computed from the committed captures / microbenchmarks, the clock sampler on ranks that do not sample."""
+rooflines computed from the committed captures / microbenchmarks, the clock sampler on ranks that do not sample, the arrays
+--dump-outputs writes."""
 import glob
 import json
 import os
@@ -8,6 +9,9 @@ from types import SimpleNamespace
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+
+import numpy as np  # noqa: E402
+import torch  # noqa: E402
 
 import bench  # noqa: E402
 import workloads as W  # noqa: E402
@@ -62,3 +66,24 @@ def test_committed_bench_lines_carry_the_contract_keys():
     assert ref["impl"] == "reference" and ref["config"] == line["config"] and ref["metric"] == line["metric"]
     gov = {r["kernel"]: r["governing"] for r in line["rooflines"]}
     assert 0.9 < gov["f2b_field_fwd_slots"]["frac"] <= 1.01 and 0.6 < gov["f2b_hash_bwd"]["frac"] < 0.95
+
+
+def test_dump_outputs_types_sampling_and_files(tmp_path):
+    """Every returned array becomes DIR/<name>.npy in float32 (integers in float64); one larger than DUMP_CAP is replaced by the
+    same seeded sample of its elements on every call."""
+    grad = lambda *shape: SimpleNamespace(grad=torch.rand(shape))
+    table = torch.rand(bench.DUMP_CAP + 5, 2)
+    prob = dict(field=SimpleNamespace(feat_pool_=SimpleNamespace(grad=table), mlp_=SimpleNamespace(params_=grad(8))),
+                shader=SimpleNamespace(mlp_=SimpleNamespace(params_=grad(4))), renderer=SimpleNamespace(app_emb_=SimpleNamespace(grad=None)))
+    res = SimpleNamespace(colors=torch.rand(6, 3), disparity=torch.rand(6), depth=torch.rand(6), first_oct_dis=torch.rand(6, 1),
+                          weights=torch.rand(20), idx_start_end=torch.arange(12, dtype=torch.int32).reshape(6, 2),
+                          edge_feats=torch.rand(4, 2, 16))
+    out = bench.step_outputs(prob, torch.tensor(0.5, requires_grad=True), res)
+    assert "grad_app_emb" not in out and out["loss"].shape == (1,) and out["colors"].shape == (6, 3)
+    assert out["idx_start_end"].dtype == np.float64 and (out["idx_start_end"] == np.arange(12).reshape(6, 2)).all()
+    assert all(a.dtype == np.float32 for k, a in out.items() if k != "idx_start_end")
+    assert out["grad_feat_pool"].shape == (bench.DUMP_CAP,) and np.isin(out["grad_feat_pool"][:100], table.numpy()).all()
+    np.testing.assert_array_equal(out["grad_feat_pool"], bench.step_outputs(prob, torch.tensor(0.5), res)["grad_feat_pool"])
+    bench.write_outputs(str(tmp_path / "d"), out)
+    assert sorted(os.listdir(tmp_path / "d")) == sorted(k + ".npy" for k in out)
+    np.testing.assert_array_equal(np.load(tmp_path / "d" / "weights.npy"), out["weights"])
