@@ -58,6 +58,7 @@ SIGNATURES = {
     "f2b_field_shade_fwd": [_P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
     "f2b_shader_mlp_rgb_fwd": [_P, _P, c_int, _P, _P, _P, _P],
     "f2b_mlp_bwd2": [_P, _P, _P, _P, _P, c_int, c_int, _P, _P, _P],
+    "f2b_field_bwd_scatter": [_P, _P, _P, c_int, _P, _P, c_int, _P, _P, _P, _P, c_int, c_int, c_float, _P, _P, _P],
     "f2b_mlp_fwd_v0": [_P, _P, c_int, c_int, _P, _P, _P],
     "f2b_mlp_bwd_v0": [_P, _P, _P, _P, c_int, c_int, _P, _P, _P],
     "f2b_mlp_fwd_tc": [_P, _P, c_int, c_int, _P, _P, _P],
@@ -173,8 +174,14 @@ def stream():
     return torch.cuda.current_stream().cuda_stream
 
 
+# The field-MLP backward and the hash scatter as one kernel (f2b_field_bwd_scatter); F2B_FIELD_BWD_SCATTER=0 restores the
+# two-kernel sequence (f2b_mlp_bwd2 -> fp16 dL/dfeatures in memory -> f2b_hash_bwd) for A/B runs.  The data-parallel level-slab
+# scatter always runs the two-kernel sequence.
+FIELD_BWD_SCATTER = os.environ.get("F2B_FIELD_BWD_SCATTER", "1") != "0"
+
 # kernels launched per entry point (for bench.py's gpu_launches claim; memsets are not counted)
-KERNELS_PER_CALL = {"f2b_render_sizeof": 0, "f2b_render_phase1": 7, "f2b_render_phase2_fwd": 10, "f2b_render_bwd": 8, "f2b_render_grad_finalize": 2,
+KERNELS_PER_CALL = {"f2b_render_sizeof": 0, "f2b_render_phase1": 7, "f2b_render_phase2_fwd": 10,
+                    "f2b_render_bwd": 5 if FIELD_BWD_SCATTER else 8, "f2b_render_grad_finalize": 2, "f2b_field_bwd_scatter": 1,
                     "f2b_sampler_count": 2, "f2b_sampler_march": 2, "f2b_sampler_march_bg": 2, "f2b_early_stop": 2, "f2b_hash_level_scales": 1, "f2b_device_info": 0,
                     "f2b_abi_version": 0, "f2b_set_mlp_impl": 0, "f2b_get_mlp_impl": 0}
 LAUNCHES = 0      # running count of product kernels launched through this binding

@@ -1,5 +1,6 @@
-// hash.cuh — device functions of the anchored hash-grid encode shared by hash.cu (stand-alone encode)
-// and field.cu (encode fused in front of the tcgen05 MLP).  See hash.cu for the design notes.
+// hash.cuh — device functions of the anchored hash-grid encode and its backward shared by hash.cu (stand-alone encode / scatter),
+// field.cu (encode fused in front of the tcgen05 MLP) and mlp_tc_bwd.cu (scatter fused behind the field-MLP backward).
+// See hash.cu for the design notes.
 #pragma once
 #include "common.cuh"
 
@@ -87,6 +88,74 @@ __device__ __forceinline__ void encode_point(const __half* __restrict__ table,
     Corner8 c;
     corners(x0, x1, x2, scales[l], prim_pool + tv * 3, bias_pool + tv * 3, (unsigned)local_size, c);
     out[l] = encode_level(table, l, local_size, c);
+  }
+}
+
+// Backward of one level for a warp that owns 32 CONSECUTIVE samples (lane i = sample i of the group).  Samples of a ray are
+// consecutive, so at the coarse levels many lanes fall into the same grid cell and hit the same 8 table entries.  Lanes are grouped
+// into runs of identical (cell, volume); when the warp has few runs, the 16 per-run sums (8 corners x 2 channels) are formed with a
+// segmented shuffle scan and only the run's last lane issues the 8 vector reductions red.global.add.v2.f32 — up to 32x fewer L2
+// atomics at the coarse levels; fine levels (every lane its own run) take the direct path.  fp32 accumulation (the reference
+// accumulates fp16 atomics of grad*128, Hash3DAnchored.cu:145-151, and casts/divides afterwards); zero-gradient rows are skipped
+// (:149) — a NaN row stays live, so a non-finite gradient still reaches the table.
+// (x0, x1, x2) = (pts + 1) / 2 and v = the volume of the lane's sample, read only on live lanes; (g0, g1) = dL/d the level's two
+// features, before grad_mul.  Shared by hash_bwd_kernel (hash.cu) and field_bwd_scatter_kernel (mlp_tc_bwd.cu).
+constexpr int kDirectHeads = 24;
+
+__device__ __forceinline__ void hash_bwd_level(int l, int lane, bool valid, float x0, float x1, float x2, int v, float g0, float g1,
+                                               const int* __restrict__ prim_pool, const float* __restrict__ bias_pool, int n_volumes,
+                                               int local_size, float grad_mul, float* __restrict__ grad_table) {
+  const bool live = valid && !(g0 == 0.f && g1 == 0.f);
+  if (!__any_sync(0xffffffffu, live)) return;
+  g0 *= grad_mul; g1 *= grad_mul;
+  Corner8 c;
+  if (live) {
+    const int tv = l * n_volumes + v;
+    corners(x0, x1, x2, level_scale(l), prim_pool + tv * 3, bias_pool + tv * 3, (unsigned)local_size, c);
+  } else {
+#pragma unroll
+    for (int k = 0; k < 8; k++) { c.idx[k] = 0; c.w[k] = 0.f; }
+    c.cell[0] = c.cell[1] = c.cell[2] = 0;
+    v = -1;
+  }
+  // run heads: key differs from the previous lane (dead lanes never merge)
+  const unsigned pcx = __shfl_up_sync(0xffffffffu, c.cell[0], 1), pcy = __shfl_up_sync(0xffffffffu, c.cell[1], 1),
+                 pcz = __shfl_up_sync(0xffffffffu, c.cell[2], 1);
+  const int prev_v = __shfl_up_sync(0xffffffffu, v, 1);       // dead lanes carry v = -1 and never merge
+  const bool head = (lane == 0) || !live || c.cell[0] != pcx || c.cell[1] != pcy || c.cell[2] != pcz || v != prev_v;
+  const unsigned heads = __ballot_sync(0xffffffffu, head);
+  float* base = grad_table + size_t(l) * local_size;
+  if (__popc(heads) > kDirectHeads) {                         // mostly singleton runs: direct reductions
+    if (live) {
+#pragma unroll
+      for (int k = 0; k < 8; k++)
+        atomicAdd(reinterpret_cast<float2*>(base + size_t(c.idx[k]) * 2), make_float2(c.w[k] * g0, c.w[k] * g1));
+    }
+    return;
+  }
+  // segmented inclusive scan within runs; the last lane of each run holds the run total
+  const unsigned below = heads & ((2u << lane) - 1u);         // heads at or below my lane
+  const int run_start = 31 - __clz(below);
+  float s[16];
+#pragma unroll
+  for (int k = 0; k < 8; k++) { s[2 * k] = c.w[k] * g0; s[2 * k + 1] = c.w[k] * g1; }
+  // only ceil(log2(longest run)) stages move data; the rest would be no-ops (warp-uniform early exit)
+  const int max_run = __reduce_max_sync(0xffffffffu, lane - run_start + 1);
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    if (o >= max_run) break;
+    const bool take = (lane - o) >= run_start;
+#pragma unroll
+    for (int k = 0; k < 16; k++) {
+      const float u = __shfl_up_sync(0xffffffffu, s[k], o);
+      if (take) s[k] += u;
+    }
+  }
+  const bool tail = (lane == 31) || ((heads >> (lane + 1)) & 1u);
+  if (live && tail) {
+#pragma unroll
+    for (int k = 0; k < 8; k++)
+      atomicAdd(reinterpret_cast<float2*>(base + size_t(c.idx[k]) * 2), make_float2(s[2 * k], s[2 * k + 1]));
   }
 }
 

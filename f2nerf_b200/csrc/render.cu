@@ -8,6 +8,7 @@
 // declared earlier in the header (same kernels, same order, same streams as f2nerf_b200/renderer.py used to issue one by one);
 // the only kernels of this file are the gradient un-scaling + finiteness flags that replace ~10 ATen passes.
 #include "common.cuh"
+#include <stdlib.h>
 
 namespace f2b {
 
@@ -49,6 +50,12 @@ using namespace f2b;
   } while (0)
 
 static inline char* off(void* p, int64_t bytes) { return reinterpret_cast<char*>(p) + bytes; }
+
+static bool field_bwd_scatter_on() {
+  static int on = -1;
+  if (on < 0) { const char* e = getenv("F2B_FIELD_BWD_SCATTER"); on = !(e && atoi(e) == 0); }
+  return on != 0;
+}
 
 extern "C" int f2b_render_sizeof(void) { return (int)sizeof(f2b_render); }       // binding self-check (layout drift = refuse to load)
 
@@ -101,6 +108,8 @@ extern "C" int f2b_render_bwd(const f2b_render* r) {
   const int64_t nk = r->n_kept, ne = 2 * int64_t(r->n_edge_pairs), nq = nk + ne;
   cudaStream_t st = as_stream(r->stream), side = as_stream(r->side_stream);
   const bool emb = r->app_emb && r->ray_emb_idx;
+  // scatter_mode 0: f2b_field_bwd_scatter unless F2B_FIELD_BWD_SCATTER=0 (the two-kernel sequence through dfeat16, for A/B runs)
+  const bool fused = r->scatter_mode == 0 && field_bwd_scatter_on();
   F2B_CUDA(cudaMemsetAsync(r->d_sparams, 0, sizeof(float) * r->n_shader_params, st), "f2b_render_bwd");
   F2B_CUDA(cudaMemsetAsync(r->d_fparams, 0, sizeof(float) * r->n_field_params, st), "f2b_render_bwd");
   F2B_CUDA(cudaMemsetAsync(r->d_table, 0, sizeof(float) * r->table_numel, st), "f2b_render_bwd");
@@ -118,8 +127,11 @@ extern "C" int f2b_render_bwd(const f2b_render* r) {
                          r->stream));
     F2B_TRY(f2b_shader_prep_bwd_f16(r->d_in16, r->d_logit, r->new_bounds, emb ? r->ray_emb_idx : nullptr, r->n_rays,
                                     1.f / r->shader_loss_scale, r->field_loss_scale, r->d_scene16, emb ? r->d_app : nullptr, r->stream));
-    F2B_TRY(f2b_mlp_bwd2(r->d_scene16, r->feat_q, r->f_hidden, nullptr, r->fparams16, 0, (int)nk, r->dfeat16, r->d_fparams, r->stream));
+    if (!fused) F2B_TRY(f2b_mlp_bwd2(r->d_scene16, r->feat_q, r->f_hidden, nullptr, r->fparams16, 0, (int)nk, r->dfeat16, r->d_fparams, r->stream));
   }
+  if (fused)                                                       // field MLP backward + scatter of both segments, one launch
+    return f2b_field_bwd_scatter(r->d_scene16, r->feat_q, r->fparams16, (int)nk, r->pts, r->anchors, (int)ne, r->e_pts, r->e_anc, r->prim,
+                                 r->bias, r->n_volumes, r->local_size, r->table_grad_mul, r->d_fparams, r->d_table, r->stream);
   if (ne > 0)
     F2B_TRY(f2b_mlp_bwd2(off(r->d_scene16, nk * 32), off(r->feat_q, nk * 64), r->f_hidden ? off(r->f_hidden, nk * 128) : nullptr, nullptr, r->fparams16, 0, (int)ne,
                          off(r->dfeat16, nk * 64), r->d_fparams, r->stream));

@@ -67,6 +67,10 @@ __device__ __forceinline__ void mma_commit(uint64_t* mbar) {
 __device__ __forceinline__ void mbar_init(uint64_t* mbar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(mbar)), "r"(count) : "memory");
 }
+// one arrival (release at CTA scope: the caller's earlier shared-memory writes are visible to the thread that waits)
+__device__ __forceinline__ void mbar_arrive(uint64_t* mbar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(mbar)) : "memory");
+}
 __device__ __forceinline__ void mbar_wait(uint64_t* mbar, uint32_t parity) {
   asm volatile(
       "{\n\t.reg .pred P1;\n\tLAB_WAIT:\n\t"

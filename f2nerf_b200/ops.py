@@ -114,6 +114,19 @@ def hash_bwd(prim_pool, bias_pool, n_volumes, local_size, pts, vol, vol_stride, 
     return grad_table
 
 
+def field_bwd_scatter(d_out16, feat16, params16, pts, anchors, e_pts, e_anc, prim_pool, bias_pool, n_volumes, local_size, grad_mul,
+                      d_params, grad_table):
+    """Field-MLP backward (0 hidden matmuls) + hash scatter in one kernel.  Rows [0, len(pts)) of d_out16 [P,16] / feat16 [P,32]
+    are samples at pts [.,3] / anchors [.,3] (volume = column 0), the rest edge points at e_pts / e_anc [.] (None when there are
+    none).  d_params and grad_table are accumulated into."""
+    n_kept, n_edge = pts.shape[0], d_out16.shape[0] - pts.shape[0]
+    if n_edge and (e_pts is None or e_pts.shape[0] != n_edge):
+        raise ValueError("field_bwd_scatter: edge rows without their edge points")
+    call("f2b_field_bwd_scatter", d_out16, feat16, params16, n_kept, pts, anchors, n_edge, e_pts, e_anc, prim_pool, bias_pool,
+         int(n_volumes), int(local_size), float(grad_mul), d_params, grad_table, stream())
+    return d_params, grad_table
+
+
 def field_fwd(table_f16, prim_pool, bias_pool, n_volumes, local_size, params_f16, pts, vol, vol_stride=1, logit_only=False,
               save=False, save_feat=None):
     """Fused hash encode + tcgen05 field MLP.  -> (out [n] or [n,16] fp32, feat16 | None, hidden | None).

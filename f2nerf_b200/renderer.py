@@ -565,8 +565,10 @@ class _FusedRenderFunction(torch.autograd.Function):
         slab_hook = getattr(renderer, "grad_slab_hook_", None)
         f_scale = field.mlp_.loss_scale_
         grad_mul = (1.0 / f_scale) * (getattr(renderer, "grad_premul_", 1.0) if slab_hook is not None else 1.0)
+        # dfeat16: the field MLP's fp16 dL/dfeatures, in memory only when the scatter is a separate kernel (level slabs, A/B runs)
+        two_kernel = slab_hook is not None or not _lib.FIELD_BWD_SCATTER
         B = dict(d_logit=f32(n_kept), d_raw=f16(n_kept, 16), d_in16=f16(n_kept, 32), d_scene16=f16(n_kept + n_edge, 16),
-                 dfeat16=f16(n_kept + n_edge, 32), d_sparams=f32(ra.n_shader_params), d_fparams=f32(ra.n_field_params),
+                 dfeat16=f16(n_kept + n_edge, 32) if two_kernel else None, d_sparams=f32(ra.n_shader_params), d_fparams=f32(ra.n_field_params),
                  d_table=renderer._table_grad_buffer(ctx.table_shape, dev),
                  nonfinite=torch.empty((2,), dtype=torch.int32, device=dev))
         if emb_on:
@@ -683,7 +685,7 @@ class _RenderFunction(torch.autograd.Function):
         nh_s, nh_f = shader.mlp_.n_hidden_matmuls, field.mlp_.n_hidden_matmuls
         f16 = lambda *sh: torch.empty(sh, dtype=torch.float16, device=dev)
         d_logit = torch.empty((n_kept,), dtype=torch.float32, device=dev)
-        d_raw, d_in16, d_scene16, dfeat16 = f16(n_kept, 16), f16(n_kept, 32), f16(n_q, 16), f16(n_q, 32)
+        d_raw, d_in16, d_scene16 = f16(n_kept, 16), f16(n_kept, 32), f16(n_q, 16)
         d_sparams, d_fparams = zeros(sparams16.numel()), zeros(fparams16.numel())
         d_table = torch.zeros_like(field.feat_pool_)
         d_app = torch.zeros_like(renderer.app_emb_) if ray_emb_idx is not None else None
@@ -714,6 +716,10 @@ class _RenderFunction(torch.autograd.Function):
             with torch.cuda.stream(side):
                 ops.hash_bwd(*hash_args, pts, anc, stride, dfeat16[s0:s1], grad_mul, d_table)
 
+        # one chunk, no slab hook: the field-MLP backward and the scatter of both segments as ONE kernel (f2b_field_bwd_scatter)
+        fused = (_lib.FIELD_BWD_SCATTER and slab_hook is None and len(ctx.cuts) == 1 and nh_f == 0
+                 and _lib.lib.f2b_get_mlp_impl() == 1)
+        dfeat16 = None if fused else f16(n_q, 32)
         for r0, r1, s0, s1 in ctx.cuts:
             if s1 <= s0:
                 continue
@@ -727,11 +733,17 @@ class _RenderFunction(torch.autograd.Function):
                  stream())
             ops.shader_prep_bwd_f16(d_in16, d_logit, bounds[r0:r1], None if ray_emb_idx is None else ray_emb_idx[r0:r1],
                                     1.0 / s_scale, f_scale, d_scene16, d_app)
+            if fused:
+                continue
             call("f2b_mlp_bwd2", d_scene16[s0:s1], feat16[s0:s1], None if f_hidden is None else f_hidden[0, s0:s1],
                  f_hidden[1, s0:s1] if (nh_f and f_hidden is not None) else None, fparams16, int(nh_f), ns, dfeat16[s0:s1], d_fparams,
                  stream())
             scatter(segments[0][0][s0:s1], segments[0][1][s0:s1], segments[0][2], s0, s1)
-        for pts_e, anc_e, stride_e, first, rows in segments[1:]:          # TV-loss edge points: field MLP + scatter only
+        if fused:
+            edge = segments[1] if len(segments) > 1 else (None, None, 1, n_kept, 0)
+            ops.field_bwd_scatter(d_scene16, feat16, fparams16, segments[0][0], segments[0][1], edge[0], edge[1], *hash_args,
+                                  grad_mul, d_fparams, d_table)
+        for pts_e, anc_e, stride_e, first, rows in ([] if fused else segments[1:]):   # TV-loss edge points: field MLP + scatter only
             if rows > 0:
                 call("f2b_mlp_bwd2", d_scene16[first:first + rows], feat16[first:first + rows],
                      None if f_hidden is None else f_hidden[0, first:first + rows],

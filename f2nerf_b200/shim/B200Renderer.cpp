@@ -70,6 +70,12 @@ bool fused_forward() {
   static const bool on = [] { const char* e = getenv("F2B_FUSED_FORWARD"); return !e || atoi(e) != 0; }();
   return on;
 }
+// F2B_FIELD_BWD_SCATTER (default 1): the field-MLP backward and the hash scatter as one kernel (f2b_field_bwd_scatter); 0 runs
+// f2b_mlp_bwd2 -> dfeat16 -> f2b_hash_bwd (the same switch as the Python host's)
+bool field_bwd_scatter() {
+  static const bool on = [] { const char* e = getenv("F2B_FIELD_BWD_SCATTER"); return !e || atoi(e) != 0; }();
+  return on;
+}
 bool validate_weights() {
   static const bool on = [] { const char* e = getenv("F2B_VALIDATE_WEIGHTS"); return !e || atoi(e) != 0; }();
   return on;
@@ -232,7 +238,7 @@ public:
     const float s_scale = shader->mlp_->loss_scale_, f_scale = field->mlp_->loss_scale_;
     Tensor d_logit = torch::empty({n_kept}, CUDAFloat);
     Tensor d_raw = torch::empty({n_kept, 16}, kHalf), d_in16 = torch::empty({n_kept, 32}, kHalf);
-    Tensor d_scene16 = torch::empty({n_q, 16}, kHalf), dfeat16 = torch::empty({n_q, 32}, kHalf);
+    Tensor d_scene16 = torch::empty({n_q, 16}, kHalf);
     Tensor d_sparams = torch::zeros({k.sparams16.numel()}, CUDAFloat), d_fparams = torch::zeros({k.fparams16.numel()}, CUDAFloat);
     const int64_t table_numel = ctx->saved_data["table_numel"].toInt();
     const int local_size = ((field->pool_size_ / N_LEVELS) >> 4) << 4;
@@ -263,14 +269,22 @@ public:
                            (int) n_kept, P(d_in16), PF(d_sparams), cur_stream()));
     F2B_CHECK(f2b_shader_prep_bwd_f16(P(d_in16), PF(d_logit), PI(k.bounds), emb_on ? PI(k.ray_emb_idx) : nullptr, n_rays,
                                       1.f / s_scale, f_scale, P(d_scene16), PF(d_app), cur_stream()));
-    F2B_CHECK(f2b_mlp_bwd2(P(d_scene16), P(k.feat16), P(k.f_hidden), nullptr, P(k.fparams16), 0, (int) n_q, P(dfeat16),
-                           PF(d_fparams), cur_stream()));
-    F2B_CHECK(f2b_hash_bwd(field->prim_pool_.data_ptr<int>(), field->bias_pool_.data_ptr<float>(), field->n_volumes_, local_size,
-                           PF(k.pts), PI(k.anchors), 3, (int) n_kept, P(dfeat16), 1, 1.f / f_scale, PF(d_table), cur_stream()));
-    if (n_q > n_kept) {
+    if (field_bwd_scatter()) {
+      F2B_CHECK(f2b_field_bwd_scatter(P(d_scene16), P(k.feat16), P(k.fparams16), (int) n_kept, PF(k.pts), PI(k.anchors),
+                                      (int) (n_q - n_kept), n_q > n_kept ? PF(k.e_pts) : nullptr, n_q > n_kept ? PI(k.e_anc) : nullptr,
+                                      field->prim_pool_.data_ptr<int>(), field->bias_pool_.data_ptr<float>(), field->n_volumes_,
+                                      local_size, 1.f / f_scale, PF(d_fparams), PF(d_table), cur_stream()));
+    } else {
+      Tensor dfeat16 = torch::empty({n_q, 32}, kHalf);
+      F2B_CHECK(f2b_mlp_bwd2(P(d_scene16), P(k.feat16), P(k.f_hidden), nullptr, P(k.fparams16), 0, (int) n_q, P(dfeat16),
+                             PF(d_fparams), cur_stream()));
       F2B_CHECK(f2b_hash_bwd(field->prim_pool_.data_ptr<int>(), field->bias_pool_.data_ptr<float>(), field->n_volumes_, local_size,
-                             PF(k.e_pts), PI(k.e_anc), 1, (int) (n_q - n_kept), (char*) P(dfeat16) + n_kept * 64, 1, 1.f / f_scale,
-                             PF(d_table), cur_stream()));
+                             PF(k.pts), PI(k.anchors), 3, (int) n_kept, P(dfeat16), 1, 1.f / f_scale, PF(d_table), cur_stream()));
+      if (n_q > n_kept) {
+        F2B_CHECK(f2b_hash_bwd(field->prim_pool_.data_ptr<int>(), field->bias_pool_.data_ptr<float>(), field->n_volumes_, local_size,
+                               PF(k.e_pts), PI(k.e_anc), 1, (int) (n_q - n_kept), (char*) P(dfeat16) + n_kept * 64, 1, 1.f / f_scale,
+                               PF(d_table), cur_stream()));
+      }
     }
     d_sparams = d_sparams / s_scale;
     d_fparams = d_fparams / f_scale;

@@ -200,6 +200,16 @@ int f2b_shader_mlp_rgb_fwd(const void* mlp_in_f16, const void* shader_params_f16
  * 96 B read + 64 B written per sample instead of 224 / 352 + 64 (and the forward does not write 128 / 256 B). */
 int f2b_mlp_bwd2(const void* dout_f16, const void* in_f16, const void* hidden0_f16, const void* hidden1_f16,
                  const void* params_f16, int n_hidden_matmuls, int n_pts, void* din_f16, float* dparams_f32, void* stream);
+/* Field-MLP backward and hash-table scatter in one kernel: f2b_mlp_bwd2(dout, in, NULL, NULL, params, 0, ...) followed by
+ * f2b_hash_bwd of its fp16 dL/dinput, without the dL/dinput rows ever reaching memory.  Rows [0, n_kept) of dout_f16 [.,16] /
+ * in_f16 [.,32] are the samples at pts [n_kept,3] with volume anchors[3*i]; rows [n_kept, n_kept + n_edge) those at e_pts
+ * [n_edge,3] with volume e_anc[i].  dparams_f32 (field MLP, 0 hidden matmuls) and grad_table [pool,2] are accumulated into;
+ * dL/dinput is multiplied by grad_mul before it is scattered.  Same dL/dinput bits and per-run sums as the two-kernel sequence;
+ * only the order of the fp32 reductions differs.  tcgen05 only. */
+int f2b_field_bwd_scatter(const void* dout_f16, const void* in_f16, const void* params_f16, int n_kept, const float* pts,
+                          const int* anchors, int n_edge, const float* e_pts, const int* e_anc, const int* prim_pool,
+                          const float* bias_pool, int n_volumes, int local_size, float grad_mul, float* dparams_f32,
+                          float* grad_table, void* stream);
 
 /* Implementation selection for f2b_mlp_fwd / f2b_mlp_bwd: 1 = tcgen05/TMEM kernels (default when
  * built), 0 = CUDA-core twin (validation).  Env F2B_MLP_IMPL overrides the default. */
@@ -366,8 +376,10 @@ int f2b_weight_var_bwd(const float* weights, const int* idx_start_end, int n_out
  *   f2b_render_phase2_fwd  compaction -> [TRAIN: edge points + their encode] -> point->camera index -> parameter casts ->
  *                          field MLP + shader-input epilogue -> edge-point MLP -> shader MLP + colour activation ->
  *                          composite                                                             (Renderer.cpp:127-208)
- *   f2b_render_bwd         zero-fills -> composite/activation bwd -> shader MLP bwd -> input-assembly bwd -> field MLP bwd
- *                          (ray samples, edge points) -> [scatter_mode 0: hash scatter of both on side_stream, joined]
+ *   f2b_render_bwd         zero-fills -> composite/activation bwd -> shader MLP bwd -> input-assembly bwd -> scatter_mode 0:
+ *                          field MLP bwd + hash scatter of ray samples and edge points in one kernel (f2b_field_bwd_scatter;
+ *                          F2B_FIELD_BWD_SCATTER=0: field MLP bwd into dfeat16, the scatter of both on side_stream, joined);
+ *                          scatter_mode 1: field MLP bwd into dfeat16 only (the caller scatters it by level slabs)
  *   f2b_render_grad_finalize  un-scale the two MLP gradients (TCNNWP.cpp:225-229) and raise the per-MLP non-finite flags
  *                          (dL/dparams, and dL/dinput through d_app / the live table gradient; TCNNWP.cpp:231-240)
  * ------------------------------------------------------------------------------------------ */
@@ -398,7 +410,7 @@ typedef struct f2b_render {
   /* backward */
   const float* d_colors; const float* d_disparity; const float* d_depth; const float* d_weights; const float* d_edge /* [2*pairs,16] */;
   float gs_progress, shader_loss_scale, field_loss_scale, table_grad_mul;
-  float* d_logit; void* d_raw; void* d_in16; void* d_scene16; void* dfeat16;
+  float* d_logit; void* d_raw; void* d_in16; void* d_scene16; void* dfeat16 /* unused (may be NULL) by the one-kernel scatter */;
   float* d_sparams; float* d_fparams; float* d_table; int64_t table_numel; int64_t table_live; float* d_app;
   int scatter_mode;                                      /* 0: scatter inside f2b_render_bwd; 1: the caller scatters (level slabs) */
   int* nonfinite;                                        /* [2] device ints: shader MLP, field MLP */
